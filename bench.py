@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """Benchmark of the C2-Matching restoration-forward hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     (N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (float32):
+`sr` = the SR batch of the device-resident forward (`value`), `e2e_sr` = the host SR batch of the end-to-end
+call (`e2e`), 19.7 MB each; rank 0's batch when N > 1; with --impl reference, `sr` of its one-image step.
+Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 Metric (BASELINE.json): SR images/s, LR 160x160 -> 640x640 with a 500x500 Ref (zero-padded to
 640x640, as the reference dataset does).  A step = one full forward (extractor -> correlation /
@@ -19,6 +24,7 @@ path on this box's physical host cores, bounded sample), parity (image 0 of the 
 that same oracle run), micro (BASELINE configs 3 and 4), clocks, gpu_launches.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -56,6 +62,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(['nvidia-smi', f'--query-gpu={self.Q}', '--format=csv,noheader,nounits', '-i',
                                           str(self.index), '-lms', '100'], stdout=subprocess.PIPE,
                                          stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)      # no sampler left running if the benchmark fails before stop()
         except Exception:
             self.proc = None
 
@@ -139,6 +146,14 @@ def cpu_baseline(pair, timed_runs=3, b4_budget_s=120.0):
     return rec, want
 
 
+def dump_outputs(out_dir, arrays):
+    """{name: tensor} -> out_dir/<name>.npy in float32 (see --dump-outputs)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------- reference arm
 def run_reference(args, rank):
     if rank != 0:
@@ -149,23 +164,19 @@ def run_reference(args, rank):
     torch.set_num_threads(threads)
     sd_e, sd_m, sd_g = seeded_weights()
     img_lq, img_up, img_ref = [t[:1] for t in synthetic_pair(1234, BATCH, LR, REF)]     # bounded sample: image 0, 1 image per step
-    budget_s = 200.0
-    t_est = None
-    for _ in range(max(1, min(args.warmup, 1))):
-        t0 = time.perf_counter()
-        ref_path.full_forward(sd_e, sd_m, sd_g, img_lq, img_up, img_ref)
-        t_est = time.perf_counter() - t0
-    steps = max(1, min(args.steps, int(budget_s / max(t_est, 1e-3))))
+    ref_path.full_forward(sd_e, sd_m, sd_g, img_lq, img_up, img_ref)         # warm-up
     t0 = time.perf_counter()
-    for _ in range(steps):
-        ref_path.full_forward(sd_e, sd_m, sd_g, img_lq, img_up, img_ref)
+    for _ in range(args.steps):
+        sr = ref_path.full_forward(sd_e, sd_m, sd_g, img_lq, img_up, img_ref)
     dt = time.perf_counter() - t0
-    v = steps / dt
-    sample = (f'1 image per step (config-2 shapes), {steps} timed steps of {args.steps} requested, '
+    v = args.steps / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'sr': sr})
+    sample = (f'1 image per step (config-2 shapes), {args.steps} timed steps after 1 warm-up, '
               f'torch-CPU oracle port of the reference path, {threads} threads = physical cores ({logical} logical)')
     print(json.dumps({
         'impl': 'reference', 'metric': 'SR images/sec (160x160->640x640, 500x500 Ref)', 'value': v, 'unit': 'images/s',
-        'n_gpus': args.gpus, 'steps': steps, 'warmup': 1, 'ms_per_step': dt / steps * 1e3, 'higher_is_better': True,
+        'n_gpus': args.gpus, 'steps': args.steps, 'warmup': 1, 'ms_per_step': dt / args.steps * 1e3, 'higher_is_better': True,
         'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': {'workload': WORKLOAD, 'reference_arm': 'CPU, batch 1 per step'},
         'cpu_baseline': {'value': v, 'unit': 'images/s', 'cores': threads, 'kind': 'port', 'sample': sample},
@@ -212,17 +223,19 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
-        """K steps, each bracketed by events on the current stream, L2 flushed (untimed) between them."""
+        """K steps, each bracketed by events on the current stream, L2 flushed (untimed) between them.
+        Returns (max-over-ranks ms, what the last step returned)."""
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
         for e0, e1 in evs:
+            out = None          # free the previous result first: each step allocates as if it had been discarded
             flush.fill_(1)
             e0.record()
-            fn()
+            out = fn()
             e1.record()
         barrier()
         ms = sum(e0.elapsed_time(e1) for e0, e1 in evs)
-        return max_over_ranks(ms, dev)
+        return max_over_ranks(ms, dev), out
 
     step_eager = lambda: pipe.forward(*devt)
     step_dev = (lambda: pipe.forward_graphed(*devt)) if args.cuda_graph else step_eager
@@ -245,16 +258,22 @@ def run_ours(args, rank, world, local_rank):
         sampler.start()
     # (1) the headline numbers: library profiling hook OFF, nothing but the step inside the events
     ops.profile_enable(False)
-    ms_dev = timed(step_dev, args.steps)
+    ms_dev, sr_dev = timed(step_dev, args.steps)
+    # copied out before anything else runs (a graph replay or a later forward may reuse the buffer); the device
+    # batch is released right away, so the passes below allocate as if it had been discarded
+    dumped = {'sr': sr_dev.cpu()} if args.dump_outputs and rank == 0 else None
+    del sr_dev
     launches = launches_per_step * args.steps
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, sr_e2e = timed(step_e2e, args.steps)       # sr_e2e is out_host, the pinned buffer every e2e step fills
+    if dumped is not None:
+        dumped['e2e_sr'] = sr_e2e.clone()
     clocks = sampler.stop() if sampler else None
     # (2) separate pass for the per-kernel-class device times (2 cudaEventRecord per launch: not part of `value`)
     prof_steps = max(1, min(args.steps, 5))
     ops.profile_enable(True)
     for k in ops.PROF_KERNELS:
         ops.profile_collect(k)
-    ms_prof = timed(step_eager, prof_steps)
+    ms_prof = timed(step_eager, prof_steps)[0]
     prof = {k: ops.profile_collect(k) for k in ops.PROF_KERNELS}
     ops.profile_enable(False)
 
@@ -342,6 +361,8 @@ def run_ours(args, rank, world, local_rank):
             'gpu_launches': int(launches), 'roofline': roofline, 'cpu_baseline': cpu, 'parity': parity, 'micro': micro,
             'clocks': clocks,
         }), flush=True)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if dist_on:
         torch.distributed.destroy_process_group()
 
@@ -440,7 +461,7 @@ def run_config5(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=None, help='timed steps of config2 (default 10)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', choices=['ours', 'reference'], default='ours')
     ap.add_argument('--tf32', type=int, default=0, help='allow cuDNN TF32 for the plain convolutions (default: exact fp32)')
@@ -459,7 +480,17 @@ def main():
     ap.add_argument('--metrics-device', choices=['cuda', 'cpu'], default='cuda',
                     help="config5: where PSNR/SSIM run ('cpu' = the reference's numpy/cv2 arithmetic on a thread pool)")
     ap.add_argument('--per-batch-workers', action='store_true', help='config5: one BATCH per loader-worker task')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='config2: write the outputs of the last timed step to DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.workload == 'config5' and args.steps is not None:
+        ap.error('--steps applies to the config2 workload (config5 times one validation pass over --pairs pairs)')
+    if args.steps is None:
+        args.steps = 10
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.workload != 'config2':
+        ap.error('--dump-outputs applies to the config2 workload')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))

@@ -15,14 +15,6 @@ for p in (ROOT, os.path.join(ROOT, 'c2-matching_b200'), os.path.join(ROOT, 'test
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box)')
-    config.addinivalue_line('markers', 'refonly: needs /root/reference (authoring container only)')
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir('/root/reference/mmsr')
-    for item in items:
-        if 'refonly' in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason='/root/reference not present'))
 
 
 @pytest.fixture(scope='session')

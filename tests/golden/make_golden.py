@@ -1,13 +1,12 @@
 #!/usr/bin/env python
 """Mint the golden fixtures in this directory from the UNMODIFIED reference code.
 
-Run in the authoring container only (needs /root/reference, which does not exist on the
-GPU box):
+Needs a checkout of the reference; the tests only read what this script writes:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --reference PATH/TO/C2-Matching [corr offsets dcn full dataset specs]
 
-The reference (yumingj/C2-Matching @ 6d60149) ships no tests or golden vectors
-(SURVEY.md §4, §8c), so parity is pinned on outputs of the reference's own Python run here
+(no fixture names: all of them).  The reference (yumingj/C2-Matching @ 6d60149) ships no tests or
+golden vectors (SURVEY.md §4, §8c), so parity is pinned on outputs of the reference's own Python run here
 on CPU, imported with three shims that do not touch its arithmetic:
   1. a stub `mmcv` (only `scandir` + the `runner` helpers the imports need),
   2. a stub top-level `_ext` whose `dcn_v2_forward` is torchvision's CPU
@@ -31,10 +30,8 @@ sys.path.insert(0, HERE)
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import seeding  # noqa: E402
 
-REF_ROOT = '/root/reference'
 
-
-def install_reference_shims():
+def install_reference_shims(ref_root):
     import torchvision
     import torchvision.models.vgg as tvgg
 
@@ -90,7 +87,7 @@ def install_reference_shims():
 
         setattr(tvgg, name, make(orig))
 
-    sys.path.insert(0, REF_ROOT)
+    sys.path.insert(0, ref_root)
 
 
 def save(name, **arrays):
@@ -295,18 +292,54 @@ def gen_dataset():
     save('dataset.npz', **out)
 
 
+def gen_specs():
+    """State-dict key -> shape of the three reference nets as the model builds them, for the hand-written
+    specs in seeding.py (RestorationNet(64, 16, 8), ContrasExtractorSep(), CorrespondenceGenerationArch(vgg19))."""
+    import json
+    from mmsr.models.archs.contras_extractor_arch import ContrasExtractorSep
+    from mmsr.models.archs.corres_generation_arch import CorrespondenceGenerationArch
+    from mmsr.models.archs.ref_restoration_arch import RestorationNet
+    out = {}
+    for n, net in (('g', RestorationNet(64, 16, 8)), ('e', ContrasExtractorSep()),
+                   ('m', CorrespondenceGenerationArch(3, 1, ['relu1_1', 'relu2_1', 'relu3_1'], 'vgg19'))):
+        out[n] = {k: list(v.shape) for k, v in net.state_dict().items()}
+    # one `"key": [shape]` entry per line, so that a change of the specs reads as a change of the lines it touches
+    nets = []
+    for n, spec in out.items():
+        entries = ',\n'.join(f'  {json.dumps(k)}: {json.dumps(v)}' for k, v in spec.items())
+        nets.append(f' {json.dumps(n)}: {{\n{entries}\n }}')
+    path = os.path.join(HERE, 'reference_specs.json')
+    with open(path, 'w') as f:
+        f.write('{\n' + ',\n'.join(nets) + '\n}\n')
+    print(f'wrote reference_specs.json: {os.path.getsize(path) / 1024:.1f} KiB')
+
+
+GENERATORS = {'corr': gen_corr, 'offsets': gen_offsets, 'dcn': gen_dcn, 'full': gen_full, 'dataset': gen_dataset,
+              'specs': gen_specs}
+
+
 def main():
+    import argparse
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--reference', required=True, help='checkout of yumingj/C2-Matching @ 6d60149')
+    ap.add_argument('fixtures', nargs='*', help=f'any of {" ".join(GENERATORS)} (default: all)')
+    args = ap.parse_args()
+    unknown = set(args.fixtures) - set(GENERATORS)
+    if unknown:
+        ap.error(f'unknown fixtures: {sorted(unknown)}')
     torch.manual_seed(0)
     torch.set_num_threads(8)
-    install_reference_shims()
-    gen_corr()
-    gen_offsets()
-    gen_dcn()
-    gen_full()
-    gen_dataset()
-    meta = f'torch {torch.__version__}; numpy {np.__version__}; reference 6d60149\n'
-    with open(os.path.join(HERE, 'VERSIONS.txt'), 'w') as f:
-        f.write(meta)
+    install_reference_shims(args.reference)
+    names = args.fixtures or list(GENERATORS)
+    for name in names:
+        GENERATORS[name]()
+    # VERSIONS.txt stamps every stored fixture, so it is only rewritten when all of them were regenerated
+    if set(names) == set(GENERATORS):
+        meta = f'torch {torch.__version__}; numpy {np.__version__}; reference 6d60149\n'
+        with open(os.path.join(HERE, 'VERSIONS.txt'), 'w') as f:
+            f.write(meta)
+    else:
+        print('VERSIONS.txt left as is: it records the versions of the last full regeneration')
 
 
 if __name__ == '__main__':

@@ -118,7 +118,7 @@ def sha(t: torch.Tensor) -> str:
 #   RestorationNet(ngf=64, n_blocks=16, groups=8)   mmsr/models/archs/ref_restoration_arch.py:30-145
 #   ContrasExtractorSep()                            mmsr/models/archs/contras_extractor_arch.py:8-59
 #   CorrespondenceGenerationArch(vgg19, relu3_1)     mmsr/models/archs/corres_generation_arch.py:14-27
-# tests/test_golden_specs.py (container only) checks them against the real reference classes.
+# tests/test_host_cpu.py checks them against the reference classes' state dicts (reference_specs.json).
 def _conv_spec(d, name, cin, cout, k=3):
     d[name + '.weight'] = (cout, cin, k, k)
     d[name + '.bias'] = (cout,)

@@ -164,26 +164,12 @@ def test_metrics_and_tensor2img():
     assert 0.99 < metrics.ssim(np.random.default_rng(0).random((32, 32)) * 255, np.random.default_rng(0).random((32, 32)) * 255) <= 1.0
 
 
-@pytest.mark.refonly
 def test_specs_equal_real_reference_classes():
-    """Container only: the hand-written key/shape specs == the reference constructors."""
-    import subprocess, sys, json
-    code = r'''
-import sys, json
-sys.path.insert(0, %r)
-import make_golden as mg
-mg.install_reference_shims()
-from mmsr.models.archs.contras_extractor_arch import ContrasExtractorSep
-from mmsr.models.archs.corres_generation_arch import CorrespondenceGenerationArch
-from mmsr.models.archs.ref_restoration_arch import RestorationNet
-out = {}
-for n, net in (('g', RestorationNet(64, 16, 8)), ('e', ContrasExtractorSep()),
-               ('m', CorrespondenceGenerationArch(3, 1, ['relu1_1', 'relu2_1', 'relu3_1'], 'vgg19'))):
-    out[n] = {k: list(v.shape) for k, v in net.state_dict().items()}
-print(json.dumps(out))
-''' % os.path.join(ROOT, 'tests', 'golden')
-    r = subprocess.run([sys.executable, '-c', code], capture_output=True, text=True, check=True)
-    got = json.loads(r.stdout.strip().splitlines()[-1])
+    """The hand-written key/shape specs == the state dicts of the reference constructors (fixture:
+    reference_specs.json, minted from the reference classes by make_golden.py)."""
+    import json
+    with open(os.path.join(ROOT, 'tests', 'golden', 'reference_specs.json')) as f:
+        got = json.load(f)
     for n, spec in (('g', seeding.spec_restoration_net()), ('e', seeding.spec_extractor()), ('m', seeding.spec_net_map())):
         assert got[n] == {k: list(v) for k, v in spec.items()}
 
